@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- forward+backward views/sec of the Gaussian-splat rasterizer hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): forward+backward views/sec @ 3M Gaussians, 1920x1080, SH degree 3,
 plus achieved HBM GB/s of the dominant kernel vs the measured peak.  One "step" = one view
@@ -19,8 +19,12 @@ Prints ONE JSON line (rank 0).  Keys are documented in DESIGN.md section "Measur
 GaussianRasterizer on the same tensors and protocol (the reference has no CPU rasterizer; its
 CUDA build is the baseline BASELINE.md section 2 names), falling back to the CPU oracle port
 when oracle/_ref is absent.
+--dump-outputs DIR writes what the last timed step computed -- the rendered image, radii and every gradient a
+caller of the rasterizer receives -- as DIR/<name>.npy (float32; see dump_outputs), so that two builds run with
+the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 import argparse
+import functools
 import json
 import math
 import os
@@ -81,7 +85,15 @@ def parse():
                     help="N>1, peer exchange: equal chunks instead of halving ones")
     ap.add_argument("--force-exchange", action="store_true",
                     help="diagnostic, N=1: run the exchange path's kernels (factor-mode backward + finalize) without NCCL")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="raster / c5: write the last timed step's image, radii and gradients to DIR/<name>.npy "
+                         f"(float32, at most {DUMP_BYTES >> 20} MB in all: larger arrays are sampled, the same elements "
+                         "in every run)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.workload not in ("raster", "c5"):
+        ap.error("--dump-outputs: only the raster and c5 workloads")
     if args.peer:
         args.exchange = "peer"
     return args
@@ -179,6 +191,24 @@ def load_peaks():
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
     except Exception:
         return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(outdir, arrays):
+    """Write each tensor of `arrays` as float32 <outdir>/<name>.npy within DUMP_BYTES in all, shared equally.  A tensor
+    over its share is replaced by a sample of its flattened elements, drawn by numpy's PCG64 from seed 0 and sorted:
+    the same elements in every run with the same arguments."""
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    share = (DUMP_BYTES // len(arrays) - 4096) // 4   # float32 elements per file; 4 KB for the .npy header
+    for name, x in arrays.items():
+        a = x.detach()
+        if a.numel() > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.numel(), share, replace=False))
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+        np.save(os.path.join(outdir, name + ".npy"), a.float().cpu().numpy())
 
 
 def _cpu_sample(job):
@@ -332,6 +362,8 @@ def main():
         if h.have_ref():
             mod = h.load_ref_module()
             use_ref = True
+        elif args.dump_outputs:
+            raise SystemExit("--dump-outputs: no reference CUDA build (oracle/_ref) to run")
         else:
             # no reference CUDA build on this box: the CPU oracle port is the reference arm
             cb = cpu_baseline(args)
@@ -401,13 +433,19 @@ def main():
             p.grad = None
         means2D.grad = None
 
-    def step_device():
-        for view in views:   # this rank's views of the batch: each backward runs its own exchange
+    def step_device(keep=None):
+        """`keep`: a dict that receives what a caller of the rasterizer gets back from this step."""
+        for v, view in zip(my_views, views):   # this rank's views of the batch: each backward runs its own exchange
             vm, pm, cp, b, g = view["dev"]
             rast = mod.GaussianRasterizer(settings(vm, pm, cp, b))
             color, radii = rast(means3D=params["means3D"], means2D=means2D, opacities=params["opacities"],
                                 shs=params["shs"], scales=params["scales"], rotations=params["rotations"])
             torch.autograd.backward(color, g)
+            if keep is not None:
+                sfx = "" if len(views) == 1 else f"_view{v}"
+                keep["color" + sfx], keep["radii" + sfx] = color.detach(), radii
+        if keep is not None:
+            keep.update({"grad_" + k: p.grad for k, p in params.items()}, grad_means2D=means2D.grad)
         zero_grads()
         return radii
 
@@ -454,12 +492,13 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(fn, steps):
+    def timed(fn, steps, last=None):
+        """ms per step of `steps` calls of fn; `last`, if given, is called instead of fn for the final step."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
-            fn()
+        for i in range(steps):
+            (last if last is not None and i == steps - 1 else fn)()
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1) / steps
@@ -505,7 +544,8 @@ def main():
         _lib.profile_read()
     launches0 = 0 if use_ref else _lib.lib.sgr_launch_count()
     t_timed0 = time.perf_counter()
-    ms = timed(step_device, args.steps)
+    dumped = {}
+    ms = timed(step_device, args.steps, last=functools.partial(step_device, keep=dumped) if args.dump_outputs else None)
     t_timed1 = time.perf_counter()
     launches = 0 if use_ref else int(_lib.lib.sgr_launch_count() - launches0)
     prof = {}
@@ -641,6 +681,8 @@ def main():
     if use_ref:
         out["cpu_baseline"] = {"value": out["value"], "unit": "views/s", "cores": 0, "kind": "reference",
                                "sample": "full workload on the GPU: the reference path has no CPU implementation"}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, dumped)
     if rank == 0:
         print(json.dumps(out))
     if dist is not None:

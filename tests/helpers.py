@@ -1,5 +1,7 @@
 """Shared test plumbing: run the same seeded scene through (a) the sugar_b200 CUDA path,
-(b) the CPU oracle, (c) the unmodified reference CUDA build in oracle/_ref (when present)."""
+(b) the CPU oracle, (c) the unmodified reference CUDA build in oracle/_ref (when present), or
+compare with what (c) computed on a B200, stored in tests/golden/reference_build.npz."""
+import hashlib
 import importlib
 import os
 import sys
@@ -8,6 +10,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+REF_GOLDEN = os.path.join(ROOT, "tests", "golden", "reference_build.npz")
+GRAD_SAMPLE, GRAD_TOP = 128, 32   # elements of each gradient kept in REF_GOLDEN: a fixed spread + the largest
 
 
 def scene_kwargs(sc, use_sh=True, use_cov_precomp=False, sh_degree=3, cov3D=None):
@@ -49,6 +53,105 @@ def load_ref_module():
     sys.modules["diff_gaussian_rasterization_ref"] = mod
     spec.loader.exec_module(mod)
     return mod
+
+
+def _numpy(x):
+    return x.detach().cpu().numpy() if hasattr(x, "detach") else np.asarray(x)
+
+
+def digest(x):
+    """sha256 of an array's shape, dtype and bytes, integer and bool arrays widened to int64 first (torch.equal compares
+    integers by value across dtypes): equal digests <=> equal integer arrays / bit-identical float arrays."""
+    a = _numpy(x)
+    a = np.ascontiguousarray(a.astype(np.int64) if a.dtype.kind in "biu" else a)
+    return hashlib.sha256(repr(a.shape).encode() + a.dtype.str.encode() + a.tobytes()).hexdigest()
+
+
+def sample_index(numel, n=GRAD_SAMPLE):
+    """n flat indices spread over [0, numel) by Fibonacci hashing: integer arithmetic, the same on every platform."""
+    k = np.arange(n, dtype=np.uint64) * np.uint64(0x9E3779B97F4A7C15)
+    return np.unique(k % np.uint64(max(numel, 1))).astype(np.int64)
+
+
+def _grad_index(numel, top):
+    return np.unique(np.concatenate([sample_index(numel), np.asarray(top, np.int64)]))
+
+
+def record_reference(rec, prefix, num_rendered=None, same=None, grads=None, grads2=None):
+    """Add to `rec` (name -> array, saved as REF_GOLDEN) what RefGolden(prefix) reads back: the sha256 digests of `same`
+    (the arrays a test holds bit-identical) and of each gradient its shape, |.|_inf, values at sample_index() and at its
+    GRAD_TOP largest elements and, given `grads2` (a second run of the reference), its run-to-run rel err."""
+    import torch
+    if num_rendered is not None:
+        rec[f"{prefix}.num_rendered"] = np.int64(num_rendered)
+    if same:
+        rec[f"{prefix}.sha256"] = np.array([(k, digest(x)) for k, x in same.items()], dtype="S64")
+    if not grads:
+        return
+    names = sorted(grads)
+    shape, stats, top, values = [], [], [], []
+    for k in names:
+        flat = grads[k].detach().reshape(-1)
+        t = flat.abs().topk(min(GRAD_TOP, flat.numel())).indices.cpu().numpy()
+        idx = torch.from_numpy(_grad_index(flat.numel(), t)).to(flat.device)
+        shape.append(list(grads[k].shape) + [-1] * (4 - grads[k].dim()))
+        stats.append((flat.abs().max().item(), rel_err(_numpy(grads2[k]), _numpy(grads[k])) if grads2 is not None else np.nan))
+        top.append(np.pad(t, (0, GRAD_TOP - t.size), constant_values=-1))
+        values.append(flat[idx].cpu().numpy())
+    rec[f"{prefix}.grads"] = np.array(names)
+    rec[f"{prefix}.grad_shape"] = np.array(shape, np.int64)
+    rec[f"{prefix}.grad_stats"] = np.array(stats, np.float64)      # |ref|_inf, run-to-run rel err
+    rec[f"{prefix}.grad_top"] = np.array(top, np.int32)
+    rec[f"{prefix}.grad_values"] = np.concatenate(values).astype(np.float32)
+
+
+_GOLDEN = {}
+
+
+class RefGolden:
+    """What the unmodified reference CUDA build computed for one test case on a B200 (written by record_reference,
+    tests/golden/make_reference_build_golden.py)."""
+
+    def __init__(self, prefix):
+        if not _GOLDEN:
+            with np.load(REF_GOLDEN) as z:
+                _GOLDEN.update((k, z[k]) for k in z.files)
+        self.prefix = prefix
+        assert any(k.startswith(prefix + ".") for k in _GOLDEN), f"{prefix} not in {REF_GOLDEN}"
+        self.digests = {n.decode(): d.decode() for n, d in self.get("sha256", np.zeros((0, 2), "S64"))}
+        self.grad_names = {str(k) for k in self.get("grads", [])}
+        self._grads, off = {}, 0
+        for i, k in enumerate(self.get("grads", [])):
+            shape = tuple(int(v) for v in self["grad_shape"][i] if v >= 0)
+            top = self["grad_top"][i]
+            idx = _grad_index(int(np.prod(shape)), top[top >= 0])
+            self._grads[str(k)] = (shape, idx, self["grad_values"][off:off + idx.size], *self["grad_stats"][i])
+            off += idx.size
+
+    def __getitem__(self, k):
+        return _GOLDEN[f"{self.prefix}.{k}"]
+
+    def get(self, k, default=None):
+        return _GOLDEN.get(f"{self.prefix}.{k}", default)
+
+    @property
+    def num_rendered(self):
+        return int(self["num_rendered"])
+
+    def same(self, k, x):
+        """x equals the reference's array k bit for bit."""
+        return digest(x) == self.digests[k]
+
+    def grad_err(self, k, g):
+        """|g - ref|_inf / |ref|_inf of gradient k over the reference's stored elements."""
+        shape, idx, values, absmax, _ = self._grads[k]
+        assert tuple(g.shape) == shape, f"grad {k}: shape {tuple(g.shape)}, reference {shape}"
+        d = np.abs(_numpy(g).reshape(-1)[idx].astype(np.float64) - values).max()
+        return float(d / max(absmax, 1e-30))
+
+    def noise(self, k):
+        """The reference's own run-to-run rel err of gradient k (fp32 atomics)."""
+        return float(self._grads[k][4])
 
 
 def to_torch(sc, device="cuda"):

@@ -1,5 +1,6 @@
 """GPU parity tests (run on the B200 box): sugar_b200 CUDA path vs
-  (1) the UNMODIFIED reference CUDA build (oracle/_ref), same tensors, same process;
+  (1) the UNMODIFIED reference CUDA build: what it computed on a B200 from the same seeded inputs
+      (tests/golden/reference_build.npz: digests of the arrays held bit-exact, sampled gradients);
   (2) the CPU oracle (oracle/raster_oracle.c).
 
 Tolerances.  Everything the reference computes before blending and every integer/index output
@@ -71,52 +72,50 @@ def _cov_from_oracle(sc):
     return fw["cov3D"].copy()
 
 
+def compared_state(radii, st, use_sh):
+    """The forward state held bit-identical to the reference build's, as {name: (array, failure message)}; per-Gaussian
+    arrays only where radii > 0 (the reference leaves the others unwritten).  `st`: _C.inspect_state of ours or
+    helpers.decode_ref_state of the reference."""
+    vis = radii > 0
+    out = {"tiles_touched": (st["tiles_touched"][vis], "tiles_touched differ"),
+           "depths": (st["depths"][vis], "depths not bit-exact"),
+           "means2D": (st["means2D"][vis], "means2D not bit-exact"),
+           "conic_opacity": (st["conic_opacity"][vis], "conic/opacity not bit-exact")}
+    if use_sh:
+        out["clamped"] = (st["clamped"][vis].bool(), "clamp flags differ")
+        out["rgb"] = (st["rgb"][vis], "SH colours not bit-exact")
+    out.update(keys=(st["keys"], "sorted 64-bit keys differ"), point_list=(st["point_list"], "sorted Gaussian ids differ"),
+               ranges=(st["ranges"], "tile ranges differ"), n_contrib=(st["n_contrib"], "n_contrib differs"),
+               final_T=(st["final_T"], "final_T not bit-exact"))
+    return out
+
+
 @pytest.mark.parametrize("case", CASES, ids=[c[0] for c in CASES])
 def test_matches_reference_build(case):
-    import torch
-    if not h.have_ref():
-        pytest.skip("oracle/_ref not built")
+    """Against what the reference build computed on the same seeded inputs (helpers.RefGolden)."""
     name, P, W, H, camera, use_sh, deg, covpre, bg = case
     from sugar_b200 import diff_gaussian_rasterization as ours, scenes
     from sugar_b200 import _C
-    ref = h.load_ref_module()
+    ref = h.RefGolden("parity." + name)
     sc = _scene(name, P, W, H, camera)
     dL = scenes.upstream_grad(W, H)
     cov3D = _cov_from_oracle(sc) if covpre else None
     opts = dict(use_sh=use_sh, sh_degree=deg, use_cov_precomp=covpre, cov3D=cov3D)
     a = h.run_module(ours, sc, bg, None, **opts)
     st = _C.inspect_state(P, W, H, a["num_rendered"], a["geom"], a["binning"], a["img"])
-    b = h.run_module(ref, sc, bg, None, **opts)
-    rs = h.decode_ref_state(b, P, W, H)
 
-    assert a["num_rendered"] == b["num_rendered"]
-    assert torch.equal(a["radii"], b["radii"]), "radii differ"
-    vis = (b["radii"] > 0)
-    assert torch.equal(st["tiles_touched"][vis], rs["tiles_touched"][vis]), "tiles_touched differ"
-    eqbits = lambda x, y: torch.equal(x.contiguous().view(torch.int32), y.contiguous().view(torch.int32))
-    assert eqbits(st["depths"][vis], rs["depths"][vis]), "depths not bit-exact"
-    assert eqbits(st["means2D"][vis], rs["means2D"][vis]), "means2D not bit-exact"
-    assert eqbits(st["conic_opacity"][vis], rs["conic_opacity"][vis]), "conic/opacity not bit-exact"
-    if use_sh:
-        assert torch.equal(st["clamped"][vis].bool(), rs["clamped"][vis].bool()), "clamp flags differ"
-        assert eqbits(st["rgb"][vis], rs["rgb"][vis]), "SH colours not bit-exact"
-    assert torch.equal(st["keys"], rs["keys"]), "sorted 64-bit keys differ"
-    assert torch.equal(st["point_list"], rs["point_list"]), "sorted Gaussian ids differ"
-    assert torch.equal(st["ranges"], rs["ranges"]), "tile ranges differ"
-    assert torch.equal(st["n_contrib"], rs["n_contrib"]), "n_contrib differs"
-    assert eqbits(st["final_T"], rs["final_T"]), "final_T not bit-exact"
-    assert eqbits(a["color"], b["color"]), "image not bit-exact"
+    assert a["num_rendered"] == ref.num_rendered
+    assert ref.same("radii", a["radii"]), "radii differ"
+    for k, (x, msg) in compared_state(a["radii"], st, use_sh).items():
+        assert ref.same(k, x), msg
+    assert ref.same("color", a["color"]), "image not bit-exact"
 
     # backward
     a = h.run_module(ours, sc, bg, dL, **opts)
-    b = h.run_module(ref, sc, bg, dL, **opts)
-    b2 = h.run_module(ref, sc, bg, dL, **opts)  # the reference's own atomics noise, run to run
-    assert set(a["grads"]) == set(b["grads"])
+    assert set(a["grads"]) == ref.grad_names
     bad, sens = [], None
-    for k in sorted(b["grads"]):
-        ga, gb, gb2 = (x["grads"][k].cpu().numpy() for x in (a, b, b2))
-        assert ga.shape == gb.shape
-        err, noise = h.rel_err(ga, gb), h.rel_err(gb2, gb)
+    for k in sorted(ref.grad_names):
+        err, noise = ref.grad_err(k, a["grads"][k]), ref.noise(k)  # noise: the reference's own atomics, run to run
         # 1e-4, except where the reference cannot reproduce itself to 2e-5 (surface-aligned
         # Gaussians with a 1e-6 axis: cancellation in the scale/rotation chain): there 5x its noise, or
         # 5x what 1e-6 relative noise on the blend accumulators (= fp32 summation order) does to this
@@ -211,15 +210,13 @@ def test_full_size_properties():
     assert bool(torch.isfinite(a["color"]).all())
     for k, g in a["grads"].items():
         assert bool(torch.isfinite(g).all()), k
-    if h.have_ref():
-        ref = h.load_ref_module()
-        b = h.run_module(ref, sc, (0, 0, 0), scenes.upstream_grad(W, H), use_sh=True, sh_degree=3)
-        assert b["num_rendered"] == R
-        assert torch.equal(a["radii"], b["radii"])
-        assert torch.equal(a["color"].view(torch.int32), b["color"].view(torch.int32)), "1M/1080p image not bit-exact"
-        for k in b["grads"]:
-            err = h.rel_err(a["grads"][k].cpu().numpy(), b["grads"][k].cpu().numpy())
-            assert err <= GRAD_RTOL, f"grad {k}: rel err {err:.3e}"
+    ref = h.RefGolden("full_size")
+    assert ref.num_rendered == R
+    assert ref.same("radii", a["radii"])
+    assert ref.same("color", a["color"]), "1M/1080p image not bit-exact"
+    for k in ref.grad_names:
+        err = ref.grad_err(k, a["grads"][k])
+        assert err <= GRAD_RTOL, f"grad {k}: rel err {err:.3e}"
 
 
 def _run_raw(mod, t, sc, bg, dL, sh_degree, shs, device="cuda"):
@@ -238,15 +235,12 @@ def _run_raw(mod, t, sc, bg, dL, sh_degree, shs, device="cuda"):
                                                 rotations=rots.grad, shs=shs.grad, means2D=means2D.grad)
 
 
-@pytest.mark.parametrize("M,deg", [(16, 3), (9, 2), (4, 1), (1, 0), (16, 1)])
-def test_sh_layouts_and_misaligned_inputs(M, deg):
-    """Stored SH count M != 16 (rows not 16-byte multiples -> 4-byte cp.async path) and inputs that start at a
-    12-byte offset (no TMA bulk copy possible -> plain staging path); forward bit-exact, grads 1e-4."""
-    import torch
-    if not h.have_ref():
-        pytest.skip("oracle/_ref not built")
-    from sugar_b200 import diff_gaussian_rasterization as ours, scenes
-    ref = h.load_ref_module()
+SH_LAYOUTS = [(16, 3), (9, 2), (4, 1), (1, 0), (16, 1)]
+
+
+def run_sh_layout(mod, M, deg):
+    """The inputs of test_sh_layouts_and_misaligned_inputs through `mod` -> (color, radii, grads)."""
+    from sugar_b200 import scenes
     P, W, H = 3001, 150, 90
     sc = scenes.make_scene(P + 1, W, H, seed=40 + M, camera="posed")
     dL = scenes.upstream_grad(W, H)
@@ -255,13 +249,22 @@ def test_sh_layouts_and_misaligned_inputs(M, deg):
     tt = {k: (v[1:] if k in ("means3D", "scales", "rotations", "opacities", "shs") else v) for k, v in t.items()}
     shs = tt["shs"][:, :M, :].contiguous() if M != 16 else tt["shs"]
     assert tt["means3D"].data_ptr() % 16 != 0
-    a = _run_raw(ours, tt, sc, (0.2, 0.1, 0.3), dL, deg, shs)
-    b = _run_raw(ref, tt, sc, (0.2, 0.1, 0.3), dL, deg, shs)
-    assert torch.equal(a[1], b[1])
-    assert torch.equal(a[0].view(torch.int32), b[0].view(torch.int32)), "image not bit-exact"
-    for k in b[2]:
-        assert a[2][k].shape == b[2][k].shape
-        err = h.rel_err(a[2][k].cpu().numpy(), b[2][k].cpu().numpy())
+    return _run_raw(mod, tt, sc, (0.2, 0.1, 0.3), dL, deg, shs)
+
+
+@pytest.mark.parametrize("M,deg", SH_LAYOUTS)
+def test_sh_layouts_and_misaligned_inputs(M, deg):
+    """Stored SH count M != 16 (rows not 16-byte multiples -> 4-byte cp.async path) and inputs that start at a
+    12-byte offset (no TMA bulk copy possible -> plain staging path); forward bit-exact, grads 1e-4 against
+    what the reference build computed on the same inputs."""
+    from sugar_b200 import diff_gaussian_rasterization as ours
+    ref = h.RefGolden(f"sh_layout.{M}_{deg}")
+    a = run_sh_layout(ours, M, deg)
+    assert ref.same("radii", a[1])
+    assert ref.same("color", a[0]), "image not bit-exact"
+    assert set(a[2]) == ref.grad_names
+    for k in ref.grad_names:
+        err = ref.grad_err(k, a[2][k])
         assert err <= GRAD_RTOL, f"grad {k}: {err:.2e}"
 
 

@@ -1,6 +1,7 @@
 """SuGaR.render_image_gaussian_rasterizer as the trainers call it (SURVEY a12): the mirror in sugar_b200/render.py
 against the arguments the reference's own wrapper produced (tests/golden/render_wrapper.npz, made by running
-sugar_model.py:2085-2294 with a recording rasterizer) rasterized by the UNMODIFIED reference CUDA build."""
+sugar_model.py:2085-2294 with a recording rasterizer) rasterized by the UNMODIFIED reference CUDA build on a B200
+(tests/golden/reference_build.npz holds the digests of its image and radii)."""
 import os
 
 import numpy as np
@@ -27,16 +28,19 @@ def test_render_wrapper_matches_reference_wrapper_plus_reference_rasterizer():
     assert float((out["radii"] > 0).float().mean()) > 0.5
     # in-kernel SH vs the python colour path: same polynomial, different evaluation order
     assert float((out["image"] - img_py).abs().max()) <= 1e-5
-    if not h.have_ref():
-        pytest.skip("oracle/_ref not built")
-    ref = h.load_ref_module()
-    st = ref.GaussianRasterizationSettings(
+    # the reference build's image / radii of the arguments the reference wrapper produced: ours rasterizes those
+    # arguments to the same bits (digests of the reference build's output in tests/golden/reference_build.npz), so the
+    # mirror is held to exactly the reference's image
+    from sugar_b200 import diff_gaussian_rasterization as ours
+    st = ours.GaussianRasterizationSettings(
         image_height=H, image_width=W, tanfovx=float(g["tanfov"][0]), tanfovy=float(g["tanfov"][1]), bg=t("bg"),
         scale_modifier=1.0, viewmatrix=t("viewmatrix"), projmatrix=t("projmatrix"), sh_degree=int(g["sh_degree"]),
         campos=t("campos"), prefiltered=False, debug=False)
     m3 = t("means3D")
-    img_ref, radii_ref = ref.GaussianRasterizer(st)(means3D=m3, means2D=torch.zeros_like(m3), opacities=t("opacities"),
-                                                    colors_precomp=t("colors_precomp"), scales=t("scales"),
-                                                    rotations=t("rotations"))
+    img_ref, radii_ref = ours.GaussianRasterizer(st)(means3D=m3, means2D=torch.zeros_like(m3), opacities=t("opacities"),
+                                                     colors_precomp=t("colors_precomp"), scales=t("scales"),
+                                                     rotations=t("rotations"))
+    ref = h.RefGolden("render")
+    assert ref.same("image", img_ref) and ref.same("radii", radii_ref), "not the reference build's image / radii"
     assert float((img_py - img_ref.permute(1, 2, 0)).abs().max()) <= 2e-5
     assert float((radii_ref == out["radii"]).float().mean()) > 0.995

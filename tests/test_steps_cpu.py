@@ -35,8 +35,9 @@ def test_coarse_sdf_step_recipe_runs_and_reaches_every_parameter():
     import bench
     import bench_workloads as bw
     from oracle import field_oracle as fo
+    before = set(sys.modules)   # other tests in this process may have imported the package themselves
     steps = bw._load_steps_without_package()
-    assert not any(m == "sugar_b200" or m.startswith("sugar_b200.") for m in sys.modules if "steps" in m)
+    assert not any(m == "sugar_b200" or m.startswith("sugar_b200.") for m in set(sys.modules) - before)
     scenes = bench.load_scenes()
     sc = scenes.make_scene(500, 64, 48, seed=0)
     cam = steps.camera_from_scene(sc, "cpu")
